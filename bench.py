@@ -62,7 +62,14 @@ def parse():
     ap.add_argument("--pipeline", default="split", choices=["split", "fused"])
     ap.add_argument("--mlp", default="fp16", choices=["fp16", "fp32"],
                     help="fp16: MLP weights as fp16 working copies (as tiny-cuda-nn), tensor-core dense kernels; fp32: FMA")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed to DIR/<name>.npy (rank 0): the depth "
+                         "and image of every ray, the loss and, when training, a fixed sample of the gradients and updated "
+                         "parameters; the inputs depend on the arguments only, so two builds can be compared file for file")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return a
 
 
 def model_kwargs(levels):
@@ -334,6 +341,36 @@ def ncu_binding():
     return json.load(open(p)) if os.path.exists(p) else {}
 
 
+DUMP_SAMPLE = 1 << 16        # --dump-outputs: entries kept of each parameter tensor larger than this
+
+
+def dump_outputs(out_dir, model, last, with_params):
+    """--dump-outputs: the arrays the last timed step handed its caller, as float32 / float64 .npy files (about 20 MB at
+    the default workload): depth [rays], image [rays, 2], loss [1] and, after a training step, grad_sample / param_sample,
+    the gradients and updated parameters of every tensor in named_parameters() order.  A tensor larger than DUMP_SAMPLE
+    contributes the entries at a seeded random set of DUMP_SAMPLE positions, the same set on every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"depth": torch.cat([d.reshape(-1) for d, _ in last["chunks"]]),
+              "image": torch.cat([i.reshape(-1, 2) for _, i in last["chunks"]])}
+    if "loss" in last:
+        arrays["loss"] = last["loss"].double().reshape(1)
+    if with_params:
+        grads, params = [], []
+        for k, p in enumerate(model.parameters()):
+            flat = p.detach().reshape(-1)
+            g = p.grad.reshape(-1) if p.grad is not None else torch.zeros_like(flat)
+            if flat.numel() > DUMP_SAMPLE:
+                pos = np.sort(np.random.default_rng(k).choice(flat.numel(), DUMP_SAMPLE, replace=False))
+                pos = torch.from_numpy(pos).to(flat.device)
+                flat, g = flat[pos], g[pos]
+            params.append(flat.float())
+            grads.append(g.float())
+        arrays["grad_sample"], arrays["param_sample"] = torch.cat(grads), torch.cat(params)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.detach().cpu().numpy())
+    log(f"outputs of the last timed step: {', '.join(f'{n} {tuple(a.shape)}' for n, a in arrays.items())} -> {out_dir}")
+
+
 def gpu_eager_baseline(levels, n_rays, dev):
     """SURVEY.md 8(d)(ii) / BASELINE.md 3 'B-gpu-eager': the reference's op graph (the oracle = its plain-torch restatement,
     pinned to the reference modules to 1e-6; the modules themselves live in /root/reference, which does not exist on the GPU
@@ -446,9 +483,13 @@ def run_b200(args):
     n_streams = max(1, min(args.streams, n_chunks))
     side = [torch.cuda.Stream(device=dev) for _ in range(n_streams)] if n_streams > 1 else []
 
+    latest = {}         # --dump-outputs: the outputs of the step that ran last (references only: no work on the device)
+
     def chunk(h, ro_d, rd_d, t, e2e, last):
         out = model.render(ro_d[None, h:h + rb], rd_d[None, h:h + rb], t, staged=False, num_steps=S_STEPS,
                            perturb=True, ray_offset=ray_off0 + h)
+        if args.dump_outputs:
+            latest["chunks"].append((out["depth_lidar"].detach(), out["image_lidar"].detach()))
         # the reference's main loss (runner.py:193-213: L1 depth, label-smoothed ray-drop MSE, intensity MSE, defaults of
         # main_lidar4d.py:70-72,88) against a synthetic ground-truth image, value + gradient in one launch
         if args.loss == "unit":       # round 1's synthetic loss (unit weights): kept as the default so that rounds compare like for like
@@ -466,6 +507,8 @@ def run_b200(args):
 
     def train_step(i, e2e, streams=True):
         ro_d, rd_d, t = inputs(i, e2e)
+        latest.clear()
+        latest["chunks"] = []
         opt.zero_grad(set_to_none=True)
         main = torch.cuda.current_stream()
         parts, outs = [], []
@@ -488,6 +531,7 @@ def run_b200(args):
                 parts.append(l)
                 outs.append(r)
         tot = torch.stack(parts).sum()
+        latest["loss"] = tot
         dp.allreduce_grads()
         if train_step.adam_events is not None:        # profile pass: time the fused Adam + staging launch pair
             ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
@@ -508,6 +552,8 @@ def run_b200(args):
         ro_d, rd_d, t = inputs(i, e2e)
         with torch.no_grad():
             out = model.render(ro_d[None], rd_d[None], t, staged=False, num_steps=S_STEPS, perturb=False, ray_offset=ray_off0)
+        latest.clear()
+        latest["chunks"] = [(out["depth_lidar"], out["image_lidar"])]
         if e2e:
             host_out[:, 0:1].copy_(out["depth_lidar"].view(-1, 1), non_blocking=True)
             host_out[:, 1:3].copy_(out["image_lidar"].view(-1, 2), non_blocking=True)
@@ -551,6 +597,8 @@ def run_b200(args):
         sampler.start()
     ms, launches = timed(False, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else {}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, latest, with_params=not infer)
     log(f"timed: {ms / args.steps:.2f} ms/step")
     step(0, True)                                  # warm the e2e path (pinned copies)
     ms_e2e, _ = timed(True, args.steps, args.warmup)

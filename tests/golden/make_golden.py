@@ -359,15 +359,130 @@ def trainer_case(seed=31):
     print(f"wrote {p}: train loss {float(out[4]):.6f}, eval loss {float(e[6]):.6f}")
 
 
+def trainer_replay_case(seed=31):
+    """tests/golden/trainer_replay.npz: the UNMODIFIED Trainer.train_step and eval_step (model/runner.py:166-434, flow
+    loss on, torch_ema stand-in, Adam) on the reference model-on-shim, and every call the Trainer made into the model:
+    its arguments, what the model returned and the torch RNG state the call left behind.  tests/test_trainer_dropin.py
+    replays these calls to tests/trainer_mirror.py and requires the Trainer's loss and predictions stored here."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import ref_stubs
+    from parity_util import small_config as parity_small_config
+    from trainer_mirror import MirrorTrainer, default_opt, default_criterion, synthetic_batch
+    from test_trainer_dropin import ReplayModel
+    runner = ref_stubs.import_reference_runner()
+    orig_cuda = torch.Tensor.cuda
+    torch.Tensor.cuda = lambda self, *a, **k: self                   # runner.py:225-247 call .cuda()
+    try:
+        orc = O.build_seeded(parity_small_config(), seed, flow_last_std=0.02)
+        ref = build_reference(SMALL)
+        ref.load_state_dict(orc.ref_state_dict(), strict=False)
+        opt = default_opt(num_frames=6, num_steps=48, near_lidar=0.0105, far_lidar=0.851, fp16=False)
+        train, ev, pcs, ground = synthetic_batch(64, frame=2, num_frames=6, seed=1)
+        real = runner.Trainer("t", opt, ref, criterion=default_criterion(), device=torch.device("cpu"), workspace=None,
+                              mute=True, fp16=False, use_checkpoint="scratch", ema_decay=0.95,
+                              optimizer=lambda m: torch.optim.Adam(m.get_params(1e-2), betas=(0.9, 0.99), eps=1e-15))
+        real.pc_list, real.pc_ground_list = pcs, ground
+        real.use_refine = False
+        fx, calls = {}, []
+
+        def recorded(kind, fn):
+            def call(*args, **kw):
+                out = fn(*args, **kw)
+                i = len(calls)
+                calls.append(kind)
+                fx[f"call{i}:kind"], fx[f"call{i}:kw"] = np.array(kind), np.array(repr(sorted(kw.items())))
+                for j, a in enumerate(args):
+                    fx[f"call{i}:arg{j}"] = a.detach().numpy().copy()
+                for k, v in out.items():
+                    if torch.is_tensor(v):
+                        fx[f"call{i}:out:{k}"] = v.detach().numpy().copy()
+                fx[f"call{i}:rng"] = torch.get_rng_state().numpy()
+                return out
+            return call
+
+        real_render, real_flow = ref.render, ref.flow
+        ref.render, ref.flow = recorded("render", real_render), recorded("flow", real_flow)
+        torch.manual_seed(3)
+        a = real.train_step(train)
+        with torch.no_grad():
+            e = real.eval_step(ev)
+        ref.render, ref.flow = real_render, real_flow
+        fx["n_calls"] = len(calls)
+        fx["train:pred_intensity"], fx["train:pred_depth"] = a[0].detach().numpy(), a[2].detach().numpy()
+        fx["train:loss"] = np.float64(a[4].item())
+        fx["eval:pred_depth"], fx["eval:loss"] = e[1].numpy(), np.float64(e[6].item())
+        # the mirror on the real model, and on the replay of the recorded calls, agrees with the Trainer
+        for model in (ref, ReplayModel(fx)):
+            mirror = MirrorTrainer(opt, model, ref_stubs.CpuChamferDist(), pc_list=pcs, pc_ground_list=ground, device=torch.device("cpu"))
+            torch.manual_seed(3)
+            b = mirror.train_step(train)
+            with torch.no_grad():
+                eb = mirror.eval_step(ev)
+            assert float(a[4]) == float(b[4]) and torch.equal(a[2], b[2]) and torch.equal(a[0], b[0])
+            assert float(e[6]) == float(eb[6]) and torch.equal(e[1], eb[1])
+    finally:
+        torch.Tensor.cuda = orig_cuda
+    p = os.path.join(ROOT, "tests", "golden", "trainer_replay.npz")
+    np.savez_compressed(p, **fx)
+    print(f"wrote {p} ({os.path.getsize(p) / 1024:.1f} KiB): {calls}, train loss {float(a[4]):.6f}, eval loss {float(e[6]):.6f}")
+
+
+def chamfer_case():
+    """tests/golden/chamfer_ref.npz: distances, indices and gradients of the reference's own chamfer kernels
+    (utils/chamfer3D/chamfer3D.cu, built by oracle/build_ref.py) on the inputs of tests/test_chamfer.py's REF_CASES.
+    Needs a GPU.  Distances and indices are kept as SHA-256 of the whole array (the test asks for bit equality) plus a
+    sample; gradients (fp32 atomics, order-dependent in the last bits) as max |g|, a projection and a sample."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import hashlib
+    from oracle import build_ref
+    from test_chamfer import REF_CASES, _clouds, chamfer_grad_probes, chamfer_grad_inputs
+    ext = build_ref.load()
+    dev = torch.device("cuda:0")
+    fx = {}
+    for b, n, m, seed, dup in REF_CASES:
+        key = f"{b}x{n}x{m}_s{seed}"
+        x1, x2 = _clouds(b, n, m, seed, dup)
+        t1, t2 = torch.from_numpy(x1).to(dev), torch.from_numpy(x2).to(dev)
+        r1, r2 = torch.zeros(b, n, device=dev), torch.zeros(b, m, device=dev)
+        j1, j2 = torch.zeros(b, n, dtype=torch.int32, device=dev), torch.zeros(b, m, dtype=torch.int32, device=dev)
+        assert ext.forward(t1, t2, r1, r2, j1, j2) == 1
+        g1, g2 = chamfer_grad_inputs(b, n, m, seed)
+        gx1, gx2 = torch.zeros_like(t1), torch.zeros_like(t2)
+        assert ext.backward(t1, t2, gx1, gx2, g1.to(dev), g2.to(dev), j1, j2) == 1
+        torch.cuda.synchronize()
+        fx[key + ":inputs"] = np.array([x1.sum(dtype=np.float64), x2.sum(dtype=np.float64),
+                                        g1.double().sum().item(), g2.double().sum().item()])
+        g = np.random.default_rng(seed)
+        for name, t in (("d1", r1), ("d2", r2), ("i1", j1), ("i2", j2)):
+            a = t.cpu().numpy().reshape(-1)
+            pos = np.sort(g.choice(a.size, min(a.size, 128), replace=False)).astype(np.int32)
+            fx[f"{key}:sha:{name}"] = np.array(hashlib.sha256(a.tobytes()).hexdigest())
+            fx[f"{key}:pos:{name}"], fx[f"{key}:val:{name}"] = pos, a[pos]
+        for name, t in (("gx1", gx1), ("gx2", gx2)):
+            a = t.cpu().numpy().reshape(-1, 3)
+            pos = np.sort(g.choice(a.shape[0], min(a.shape[0], 128), replace=False)).astype(np.int32)
+            fx[f"{key}:pos:{name}"], fx[f"{key}:val:{name}"] = pos, a[pos]
+            fx[f"{key}:max:{name}"] = np.float64(np.abs(a).max())
+            fx[f"{key}:proj:{name}"] = np.float64(a.reshape(-1).astype(np.float64) @ chamfer_grad_probes(a.size))
+    p = os.path.join(ROOT, "tests", "golden", "chamfer_ref.npz")
+    np.savez_compressed(p, **fx)
+    print(f"wrote {p} ({os.path.getsize(p) / 1024:.1f} KiB)")
+
+
 if __name__ == "__main__":
     torch.set_num_threads(8)
+    if "--chamfer" in sys.argv:
+        chamfer_case()
+        sys.exit(0)
     if "--trainer-only" in sys.argv:
         trainer_case()
+        trainer_replay_case()
         rays_case()
         unet_case()
         sys.exit(0)
     hash_index_vectors()
     trainer_case()
+    trainer_replay_case()
     rays_case()
     unet_case()
     # interior frame (both neighbours), perturb off

@@ -2,17 +2,12 @@
 stand-ins for the third-party modules that are not installed here (SURVEY.md 8(c): torch_ema, tensorboardX, imageio,
 open3d; lpips / skimage are only needed by utils/metrics.py, which the Trainer class itself does not import) and for
 the chamfer extension wrapper, whose module-level `importlib.find_loader` no longer exists in Python 3.12."""
-import os
 import sys
 import types
 
 import torch
 
 REF = "/root/reference"
-
-
-def have_reference() -> bool:
-    return os.path.exists(os.path.join(REF, "model", "runner.py"))
 
 
 class _CpuChamferFn(torch.autograd.Function):

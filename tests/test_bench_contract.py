@@ -1,9 +1,13 @@
-"""bench.py contract pieces that can be checked without a GPU: the reference arm (CPU oracle port) prints the
-required JSON line on rank 0 and stays silent on the other ranks; the GPU arm refuses to run without CUDA."""
+"""bench.py contract pieces: the reference arm (CPU oracle port) prints the required JSON line on rank 0 and stays silent
+on the other ranks; the GPU arm refuses to run without CUDA; on a GPU, --dump-outputs writes the last timed step's
+outputs and repeats them from run to run."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -38,7 +42,6 @@ def test_executed_red_count_of_the_static_scatter():
     """bench.py's RED-rate binding of k_bwd_scatter_static uses the reductions the kernel EXECUTES: 8 per level, and at the
     warp-aggregated levels 8 per run of consecutive samples that share a cell (host-side run statistics of the rays)."""
     sys.path.insert(0, ROOT)
-    import numpy as np
     import bench
     from lidar4d_b200.geometry import FieldConfig
     from lidar4d_b200.rays import synthetic_sweep
@@ -75,3 +78,30 @@ def test_committed_bench_line_carries_the_contract_keys():
     assert abs(sum(v["avg_ms"] for k, v in ks.items() if "adam" not in k) * 4 - line["ms_per_step"]) < 0.03 * line["ms_per_step"]
     b = ks["k_bwd_scatter_static"]["binding"]
     assert b["frac"] <= 1.0 and b["red_lane_ops_per_sample_executed"] < b["red_lane_ops_per_sample_algorithmic"]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_last_timed_step(tmp_path):
+    """--dump-outputs writes what the last timed step computed as float32 / float64 .npy files within 64 MB, and two runs
+    with the same arguments start from the same inputs: the first step's forward outputs agree, its gradients agree up to
+    the re-ordering of fp32 atomics."""
+    args = ("--rays", "2048", "--ray-batch", "1024", "--levels", "8", "--steps", "1", "--warmup", "0", "--eager-rays", "0",
+            "--no-cpu-baseline")
+    runs = []
+    for k in range(2):
+        out = tmp_path / f"run{k}"
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args, "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=900, env=dict(os.environ, RANK="0", WORLD_SIZE="1"))
+        assert r.returncode == 0, r.stderr[-800:]
+        line = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+        assert line["steps"] == 1 and line["warmup"] == 0
+        runs.append({f[:-len(".npy")]: np.load(out / f) for f in os.listdir(out)})
+    a, b = runs
+    assert set(a) == {"depth", "image", "loss", "grad_sample", "param_sample"}
+    assert a["depth"].shape == (2048,) and a["image"].shape == (2048, 2) and a["loss"].shape == (1,)
+    assert a["grad_sample"].shape == a["param_sample"].shape
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values()) and sum(v.nbytes for v in a.values()) <= 64 << 20
+    assert all(np.isfinite(v).all() for v in a.values()) and np.abs(a["grad_sample"]).max() > 0
+    for k in ("depth", "image", "loss"):
+        assert np.abs(a[k] - b[k]).max() <= 1e-6 * np.abs(b[k]).max(), k
+    assert np.abs(a["grad_sample"] - b["grad_sample"]).max() <= 1e-4 * np.abs(b["grad_sample"]).max()

@@ -107,14 +107,6 @@ def test_chamfer_properties_full_size():
 
 
 # ---- the reference's OWN kernel (utils/chamfer3D/chamfer3D.cu compiled in place for sm_100a by oracle/build_ref.py) -------
-def _ref_ext():
-    from oracle import build_ref
-    if not os.path.exists(build_ref.so_path()):
-        # the reference sources exist only in the build container; the GPU box gets the prebuilt .so with the repo snapshot
-        pytest.skip("oracle/_ref/chamfer_3D_ref.so was not shipped to this box (built by oracle/build_ref.py where /root/reference exists)")
-    return build_ref.load()
-
-
 def test_reference_extension_was_built():
     """oracle/_ref/chamfer_3D_ref.so is the reference's chamfer extension built by the committed recipe; it travels to
     the GPU box with the snapshot (the GPU box has no /root/reference)."""
@@ -126,6 +118,26 @@ def test_reference_extension_was_built():
 
 
 REF_CASES = CASES + [(1, 4096, 4096, 11, True), (1, 60000, 50000, 12, False), (2, 1, 1, 13, False)]
+REF_GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "chamfer_ref.npz")
+
+
+def chamfer_grad_inputs(b, n, m, seed):
+    """Upstream gradients of dist1 / dist2 fed to both backward kernels."""
+    g = torch.Generator().manual_seed(seed)
+    return torch.randn(b, n, generator=g), torch.randn(b, m, generator=g)
+
+
+def chamfer_grad_probes(size):
+    """Fixed vector the stored gradients are projected on (no RNG: the same on every machine)."""
+    return np.cos(np.arange(size, dtype=np.float64) * 0.618)
+
+
+def _assert_bit_exact(fx, key, name, got):
+    import hashlib
+    a = np.ascontiguousarray(got).reshape(-1)
+    pos = fx[f"{key}:pos:{name}"]
+    assert np.array_equal(a[pos], fx[f"{key}:val:{name}"]), f"{name}: sampled entries differ from the reference kernel's"
+    assert hashlib.sha256(a.tobytes()).hexdigest() == str(fx[f"{key}:sha:{name}"]), f"{name}: differs from the reference kernel's"
 
 
 @pytest.mark.gpu
@@ -133,27 +145,30 @@ REF_CASES = CASES + [(1, 4096, 4096, 11, True), (1, 60000, 50000, 12, False), (2
 def test_chamfer_bit_exact_against_reference_kernel(b, n, m, seed, dup):
     """Distances AND indices of l4d_chamfer_forward equal NmDistanceKernel's (chamfer3D.cu:11-133) bit for bit - also on
     exact duplicates (ties -> smallest index) - and the gradients equal NmDistanceGradKernel's (:154-174) to fp32
-    atomics re-ordering.  This pins oracle/chamfer_oracle.py's assumed fma contraction as well."""
+    atomics re-ordering.  This pins oracle/chamfer_oracle.py's assumed fma contraction as well.  The reference kernels'
+    outputs on these inputs are stored in tests/golden/chamfer_ref.npz (make_golden.py --chamfer): distances and indices
+    as a SHA-256 of the whole array, gradients as max |g|, a projection and a sample of points."""
     from lidar4d_b200.chamfer import chamfer_3DDist
-    ext = _ref_ext()
+    fx = np.load(REF_GOLDEN, allow_pickle=False)
+    key = f"{b}x{n}x{m}_s{seed}"
     dev = torch.device("cuda:0")
     x1, x2 = _clouds(b, n, m, seed, dup)
+    g1, g2 = chamfer_grad_inputs(b, n, m, seed)
+    inputs = np.array([x1.sum(dtype=np.float64), x2.sum(dtype=np.float64), g1.double().sum().item(), g2.double().sum().item()])
+    assert np.array_equal(inputs, fx[key + ":inputs"]), "the test inputs are not the ones the golden outputs were made from"
     t1 = torch.from_numpy(x1).to(dev).requires_grad_(True)
     t2 = torch.from_numpy(x2).to(dev).requires_grad_(True)
     d1, d2, i1, i2 = chamfer_3DDist()(t1, t2)
-    r1, r2 = torch.zeros(b, n, device=dev), torch.zeros(b, m, device=dev)
-    j1, j2 = torch.zeros(b, n, dtype=torch.int32, device=dev), torch.zeros(b, m, dtype=torch.int32, device=dev)
-    assert ext.forward(t1.detach(), t2.detach(), r1, r2, j1, j2) == 1        # dist_chamfer_3D.py:52
-    torch.cuda.synchronize()
-    assert torch.equal(d1.detach(), r1) and torch.equal(d2.detach(), r2)
-    assert torch.equal(i1, j1) and torch.equal(i2, j2)
+    for name, t in (("d1", d1), ("d2", d2), ("i1", i1), ("i2", i2)):
+        _assert_bit_exact(fx, key, name, t.detach().cpu().numpy())
     o1, o2, oi1, oi2 = CO.chamfer_forward(x1, x2)                            # the numpy oracle agrees with the real kernel
-    assert np.array_equal(r1.cpu().numpy(), o1) and np.array_equal(j2.cpu().numpy(), oi2)
-    g = torch.Generator().manual_seed(seed)
-    g1, g2 = torch.randn(b, n, generator=g).to(dev), torch.randn(b, m, generator=g).to(dev)
-    ((d1 * g1).sum() + (d2 * g2).sum()).backward()
-    gx1, gx2 = torch.zeros_like(t1), torch.zeros_like(t2)
-    assert ext.backward(t1.detach(), t2.detach(), gx1, gx2, g1, g2, j1, j2) == 1   # dist_chamfer_3D.py:70-72
-    torch.cuda.synchronize()
-    for got, ref in ((t1.grad, gx1), (t2.grad, gx2)):
-        assert float((got - ref).abs().max()) <= 1e-5 * float(ref.abs().max()) + 1e-12
+    _assert_bit_exact(fx, key, "d1", o1)
+    _assert_bit_exact(fx, key, "i2", oi2)
+    ((d1 * g1.to(dev)).sum() + (d2 * g2.to(dev)).sum()).backward()
+    for name, got in (("gx1", t1.grad), ("gx2", t2.grad)):
+        a = got.cpu().numpy().reshape(-1, 3)
+        tol = 1e-5 * float(fx[f"{key}:max:{name}"]) + 1e-12
+        assert abs(float(np.abs(a).max()) - float(fx[f"{key}:max:{name}"])) <= tol, name
+        assert float(np.abs(a[fx[f"{key}:pos:{name}"]] - fx[f"{key}:val:{name}"]).max()) <= tol, name
+        probes = chamfer_grad_probes(a.size)
+        assert abs(float(a.reshape(-1).astype(np.float64) @ probes) - float(fx[f"{key}:proj:{name}"])) <= tol * np.abs(probes).sum(), name

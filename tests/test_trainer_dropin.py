@@ -1,11 +1,13 @@
 """Drop-in of lidar4d_b200.LiDAR4D under the reference's Trainer (VERDICT r1 #7, SURVEY.md 8(b)).
 
-The real `Trainer` (/root/reference/model/runner.py) exists only in the build container (no GPU); the CUDA module only
-runs on the GPU box (no /root/reference).  So the chain is:
-  (here, CPU)   unmodified Trainer.train_step / eval_step on the reference model-on-shim  ==  tests/trainer_mirror.py
-  (GPU box)     the mirror drives lidar4d_b200.LiDAR4D + lidar4d_b200.chamfer + lidar4d_b200.optim.Adam through
+The reference's `Trainer` (model/runner.py) is not part of this repository, and it cannot drive the CUDA module itself
+(it needs the reference's tiny-cuda-nn model code).  So the chain is:
+  (CPU)         tests/trainer_mirror.py returns the loss and predictions of the unmodified Trainer.train_step / eval_step
+                when it gets the same model answers: tests/golden/trainer_replay.npz holds the Trainer's results and every
+                call it made into the reference model-on-shim (written by tests/golden/make_golden.py)
+  (GPU)         the mirror drives lidar4d_b200.LiDAR4D + lidar4d_b200.chamfer + lidar4d_b200.optim.Adam through
                 train iterations with autocast + GradScaler + flow loss, EMA evaluate (copy_to / restore through .data),
-                a checkpoint round trip, and reproduces the loss the REAL Trainer computed here on the same parameters
+                a checkpoint round trip, and reproduces the loss the REAL Trainer computed on the CPU on the same parameters
                 (tests/golden/trainer_step.npz, written by tests/golden/make_golden.py)."""
 import io
 import os
@@ -15,7 +17,7 @@ import pytest
 import torch
 
 import ref_stubs
-from trainer_mirror import MirrorTrainer, default_opt, default_criterion, synthetic_batch
+from trainer_mirror import MirrorTrainer, default_opt, synthetic_batch
 from parity_util import small_config, cuda_model_from_oracle, rel_err
 from oracle import lidar4d_oracle as O
 
@@ -27,38 +29,58 @@ def _opt():
     return default_opt(num_frames=6, num_steps=S_SMALL, near_lidar=0.0105, far_lidar=0.851, fp16=False)
 
 
-@pytest.mark.skipif(not ref_stubs.have_reference(), reason="needs /root/reference (build container)")
-def test_mirror_reproduces_reference_trainer(monkeypatch):
-    import sys
-    sys.path.insert(0, os.path.join(GOLD))
-    import make_golden as MG
-    runner = ref_stubs.import_reference_runner()
-    monkeypatch.setattr(torch.Tensor, "cuda", lambda self, *a, **k: self)         # runner.py:225-247 call .cuda()
-    orc = O.build_seeded(small_config(), 31, flow_last_std=0.02)
-    ref = MG.build_reference(MG.SMALL)
-    ref.load_state_dict(orc.ref_state_dict(), strict=False)
+class ReplayModel:
+    """Stands in for the reference model-on-shim: answers the k-th render / flow call with what the model returned to
+    the real Trainer on its k-th call (tests/golden/trainer_replay.npz), after checking that the call carries the same
+    arguments, and leaves the torch RNG where that call left it."""
+
+    def __init__(self, fx):
+        self.fx, self.n = fx, 0
+
+    def _call(self, kind, args, kw):
+        i, fx = self.n, self.fx
+        self.n += 1
+        assert i < int(fx["n_calls"]) and str(fx[f"call{i}:kind"]) == kind, f"call {i}: unexpected {kind}"
+        assert repr(sorted(kw.items())) == str(fx[f"call{i}:kw"]), f"call {i} ({kind}): keyword arguments differ"
+        for j, a in enumerate(args):
+            assert torch.equal(a.detach().cpu(), torch.from_numpy(fx[f"call{i}:arg{j}"])), f"call {i} ({kind}): argument {j} differs"
+        torch.set_rng_state(torch.from_numpy(fx[f"call{i}:rng"]))
+        pre = f"call{i}:out:"
+        return {k[len(pre):]: torch.from_numpy(fx[k]) for k in fx.keys() if k.startswith(pre)}
+
+    def render(self, rays_o, rays_d, time, **kw):
+        return self._call("render", (rays_o, rays_d, time), kw)
+
+    def flow(self, x, time):
+        return self._call("flow", (x, time), {})
+
+
+def test_mirror_reproduces_reference_trainer():
+    """The mirror's train_step / eval_step return the loss and predictions of the UNMODIFIED Trainer, given the same
+    model answers (the recorded calls of the Trainer into the reference model-on-shim, make_golden.py)."""
+    from trainer_mirror import MirrorEMA
+    fx = np.load(os.path.join(GOLD, "trainer_replay.npz"), allow_pickle=False)
     opt = _opt()
     train, ev, pcs, ground = synthetic_batch(64, frame=2, num_frames=6, seed=1)
-    real = runner.Trainer("t", opt, ref, criterion=default_criterion(), device=torch.device("cpu"), workspace=None,
-                          mute=True, fp16=False, use_checkpoint="scratch", ema_decay=0.95,
-                          optimizer=lambda m: torch.optim.Adam(m.get_params(1e-2), betas=(0.9, 0.99), eps=1e-15))
-    real.pc_list, real.pc_ground_list = pcs, ground
-    mirror = MirrorTrainer(opt, ref, ref_stubs.CpuChamferDist(), pc_list=pcs, pc_ground_list=ground, device=torch.device("cpu"))
-    torch.manual_seed(3)
-    a = real.train_step(train)
+    model = ReplayModel(fx)
+    mirror = MirrorTrainer(opt, model, ref_stubs.CpuChamferDist(), pc_list=pcs, pc_ground_list=ground, device=torch.device("cpu"))
     torch.manual_seed(3)
     b = mirror.train_step(train)
-    assert float(a[4]) == pytest.approx(float(b[4]), rel=1e-6)
-    assert torch.allclose(a[2], b[2]) and torch.allclose(a[0], b[0])
-    real.use_refine = False
+    assert float(fx["train:loss"]) == pytest.approx(float(b[4]), rel=1e-6)
+    assert torch.allclose(torch.from_numpy(fx["train:pred_depth"]), b[2])
+    assert torch.allclose(torch.from_numpy(fx["train:pred_intensity"]), b[0])
     with torch.no_grad():
-        ea, eb = real.eval_step(ev), mirror.eval_step(ev)
-    assert float(ea[6]) == pytest.approx(float(eb[6]), rel=1e-6) and torch.allclose(ea[1], eb[1])
-    # the EMA stand-in is what both use; its arithmetic against the closed form
-    real.ema.update()
+        eb = mirror.eval_step(ev)
+    assert float(fx["eval:loss"]) == pytest.approx(float(eb[6]), rel=1e-6)
+    assert torch.allclose(torch.from_numpy(fx["eval:pred_depth"]), eb[1])
+    assert model.n == int(fx["n_calls"]), "the mirror made fewer model calls than the Trainer"
+    # the EMA stand-in the Trainer used (runner.py:98-101 through ref_stubs); its arithmetic against the closed form
+    orc = O.build_seeded(small_config(), 31, flow_last_std=0.02)
+    ema = MirrorEMA(orc.parameters(), 0.95)
+    ema.update()
     d = min(0.95, 2 / 11)
-    p0 = next(p for p in ref.parameters() if p.requires_grad)
-    assert torch.allclose(real.ema.shadow[0], p0.detach())            # shadow == param while param has not moved
+    p0 = next(p for p in orc.parameters() if p.requires_grad)
+    assert torch.allclose(ema.shadow[0], p0.detach())                 # shadow == param while param has not moved
     assert d == pytest.approx(2 / 11)
 
 

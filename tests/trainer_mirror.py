@@ -2,10 +2,11 @@
 that CALL the hot path, so that the drop-in can be exercised on the GPU box, where /root/reference does not exist
 (and the build container, where it does, has no GPU - the real Trainer and the CUDA module can never meet here).
 
-Pinned the same way as the oracle: tests/test_trainer_dropin.py::test_mirror_reproduces_reference_trainer runs the
-UNMODIFIED `Trainer.train_step` / `eval_step` (imported from /root/reference with stubs for the third-party modules
-that are not installed: torch_ema, tensorboardX, imageio, open3d; chamfer -> a CPU autograd restatement) on the
-reference model-on-shim on the CPU and requires this mirror to return the same loss and predictions.
+Pinned the same way as the oracle: tests/golden/make_golden.py runs the UNMODIFIED `Trainer.train_step` / `eval_step`
+(with stubs for the third-party modules that are not installed: torch_ema, tensorboardX, imageio, open3d; chamfer -> a
+CPU autograd restatement) on the reference model-on-shim on the CPU and stores their results together with every call
+they made into the model (tests/golden/trainer_replay.npz); tests/test_trainer_dropin.py::
+test_mirror_reproduces_reference_trainer replays those calls to this mirror and requires the same loss and predictions.
 
 Restated (file:line into /root/reference):
   train_step         model/runner.py:166-377   (main loss :179-213, CD loss :215-220, flow loss :222-254)
